@@ -23,6 +23,10 @@ BASELINE.json shapes (configs[2] mixed 2k-20k / bw 400 + rescue, configs[3] dire
 
     python bench.py --workload mixed --queue --reads R       strong scaling over a shared
                                                              NCCL-free queue of length buckets
+
+`--dump-outputs DIR` writes what the last resident timed step computed for every workload run
+(a seeded sample of its reads) as DIR/<workload>_<field>.npy in float64; the inputs depend only
+on the arguments, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -31,6 +35,9 @@ import subprocess
 import sys
 import threading
 import time
+
+# the tree may be read-only and is never written: no bytecode caches next to the sources
+sys.dont_write_bytecode = True
 
 # the CPU arms run one single-threaded worker process per host thread (the reference's
 # --processes model): keep BLAS / OpenMP pools from oversubscribing the cores
@@ -507,8 +514,60 @@ def traffic_per_read():
     return t.get('dram_bytes_per_read'), t.get('capture', 'ncu --set full')
 
 
+DUMP_VALUES_PER_CONFIG = 1 << 20     # per workload; at most 4 workloads stay under 64 MB
+DUMP_MAX_READS = 16384
+DUMP_MAX_POSITIONS = 65536
+
+
+def dump_outputs(directory, name, ctx, out, llr):
+    """Write a seeded sample of what the last batch_compute returned as float64 .npy files
+    DIR/<name>_<field>.npy: whole reads, drawn in a fixed order until DUMP_VALUES_PER_CONFIG
+    values (their per-read fields, segs, norm_mean and LLR sites), and for the LLR workload a
+    fixed sample of the finalized region statistics.  read_index holds the sampled reads.
+    Values the library leaves undefined are written as 0 so that every file is finite: the
+    float fields of a failed read (status != 0; its score is NaN) and frac / damp_frac of a
+    position without valid calls (valid_cov == 0; NaN as in the reference).  A NaN anywhere
+    else is kept."""
+    seg_off, base_off = out['seg_off'], out['base_off']
+    n = seg_off.shape[0] - 1
+    cost = np.diff(seg_off) + np.diff(base_off) + 11      # + read_index and 10 per-read values
+    if llr:
+        llr_val, llr_pos, site_off = ctx.batch_llr_download()
+        cost = cost + 2 * np.diff(site_off)
+    order = np.random.RandomState(2024).permutation(n)
+    take = np.sort(order[np.cumsum(cost[order]) <= DUMP_VALUES_PER_CONFIG][:DUMP_MAX_READS])
+
+    def ragged(a, off):
+        return np.concatenate([a[:0]] + [a[off[i]:off[i + 1]] for i in take])
+    arrays = {'read_index': take}
+    for f in ('status', 'n_iters', 'flags', 'read_start_rel_to_raw', 'sig_match_score',
+              'scale_values'):
+        arrays[f] = out[f][take]
+    arrays['segs'] = ragged(out['segs'], seg_off)
+    arrays['norm_mean'] = ragged(out['norm_mean'], base_off)
+    failed = arrays['status'] != 0
+    arrays['sig_match_score'][failed] = 0.0
+    arrays['scale_values'][failed] = 0.0
+    arrays['norm_mean'][np.repeat(failed, np.diff(base_off)[take])] = 0.0
+    if llr:
+        arrays['llr'] = ragged(llr_val, site_off)
+        arrays['llr_pos'] = ragged(llr_pos, site_off)
+        reg = ctx.region_stats_finalize(2, 0)
+        m = reg['pos'].shape[0]
+        pick = np.sort(np.random.RandomState(2025).choice(m, min(m, DUMP_MAX_POSITIONS),
+                                                          replace=False))
+        for f, v in reg.items():
+            arrays['region_' + f] = v[pick]
+        no_valid = arrays['region_valid_cov'] == 0
+        arrays['region_frac'][no_valid] = 0.0
+        arrays['region_damp_frac'][no_valid] = 0.0
+    os.makedirs(directory, exist_ok=True)
+    for f, a in arrays.items():
+        np.save(os.path.join(directory, '%s_%s.npy' % (name, f)), np.asarray(a, dtype=np.float64))
+
+
 def run_config(name, n_reads, steps, warmup, ctx, rank, local, dist, n_gpus, pin, do_parity=True,
-               int16_e2e=False):
+               int16_e2e=False, dump_dir=None):
     """warm-up, timed resident region (device clock), timed end-to-end region (host buffers),
     parity sample -- for one workload.  Returns the fields of the JSON line."""
     from tombo_b200 import _lib, synthetic as syn
@@ -584,6 +643,8 @@ def run_config(name, n_reads, steps, warmup, ctx, rank, local, dist, n_gpus, pin
     clocks = sampler.stop()
     launches_timed = ctx.launch_count() - launches0
     ctx.batch_download(out=out)
+    if dump_dir is not None:
+        dump_outputs(dump_dir, name, ctx, out, llr)
     n_ok = int((out['status'] == 0).sum())
     n_rescued = int(((out['flags'] & 2) != 0).sum())
     # ---- timed region B: end to end through the C ABI with host buffers ----
@@ -832,7 +893,8 @@ def main():
                     help='headline workload (default c1 = BASELINE configs[1])')
     ap.add_argument('--extras', default='mixed,rna,c5',
                     help='extra configs reported under extra_configs (N = 1 only); "" = none')
-    ap.add_argument('--extra-steps', type=int, default=3)
+    ap.add_argument('--extra-steps', type=int, default=None,
+                    help='timed steps of each extra config (default: --steps)')
     ap.add_argument('--no-parity', action='store_true')
     ap.add_argument('--no-int16', action='store_true')
     ap.add_argument('--queue', action='store_true', help='strong scaling over a shared work queue')
@@ -844,7 +906,15 @@ def main():
     ap.add_argument('--bucket-samples', type=int, default=60_000_000)
     ap.add_argument('--cpu-leg', default='', help=argparse.SUPPRESS)
     ap.add_argument('--cpu-scale', type=float, default=1.0, help=argparse.SUPPRESS)
+    ap.add_argument('--dump-outputs', metavar='DIR', default='',
+                    help='write a seeded sample of the last timed step\'s results to DIR/*.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.extra_steps is None:
+        args.extra_steps = args.steps
+    if args.dump_outputs and (args.queue or args.impl == 'reference'):
+        ap.error('--dump-outputs applies to the GPU path without --queue')
 
     if args.cpu_leg:                      # child: the CPU legs in a clean interpreter
         names = [n for n in args.cpu_leg.split(',') if n]
@@ -908,8 +978,10 @@ def main():
     def free_pinned():
         while pinned:
             pinned.pop().free()
+    dump_dir = args.dump_outputs if (args.dump_outputs and rank == 0) else None
     line = run_config(args.workload, n_reads, args.steps, args.warmup, ctx, rank, local, dist,
-                      args.gpus, pin, do_parity=not args.no_parity, int16_e2e=not args.no_int16)
+                      args.gpus, pin, do_parity=not args.no_parity, int16_e2e=not args.no_int16,
+                      dump_dir=dump_dir)
     free_pinned()
     if rank == 0:
         line['config']['numa'] = numa
@@ -922,7 +994,8 @@ def main():
     for e in extras:
         try:
             r = run_config(e, CONFIGS[e]['reads'], args.extra_steps, max(3, min(args.warmup, 3)),
-                           ctx, rank, local, dist, args.gpus, pin, do_parity=not args.no_parity)
+                           ctx, rank, local, dist, args.gpus, pin, do_parity=not args.no_parity,
+                           dump_dir=dump_dir)
             r['name'] = e
             if leg is not None and e in leg:
                 r['cpu_baseline'] = cpu_baseline_obj(leg, e)

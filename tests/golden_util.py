@@ -1,4 +1,5 @@
 """Helpers to replay tests/golden/*.npz (outputs of the unmodified reference)."""
+import hashlib
 import os
 
 import numpy as np
@@ -70,3 +71,45 @@ def expected(g, i):
                 read_start_rel_to_raw=int(s[5]) if not np.isnan(s[5]) else None,
                 calls=int(s[6]), rescued=bool(s[7]), n_iters=int(s[8]),
                 norm_params_changed=bool(s[9]))
+
+
+def digest(value):
+    """16-byte SHA-256 prefix of repr(value): a golden for outputs too large to store whole.
+    Callers pass plain Python values (str, int, float, lists, tuples), whose repr is exact."""
+    return np.frombuffer(hashlib.sha256(repr(value).encode()).digest()[:16], dtype=np.uint8)
+
+
+def trim_cases():
+    """3000 seeded argument sets for trim_seq_and_means: (seq, means, args)."""
+    rs = np.random.RandomState(3)
+    for _ in range(3000):
+        K = int(rs.choice([5, 6, 7])); cp = int(rs.randint(0, K))
+        L = int(rs.randint(K, 40))
+        seq = ''.join(rs.choice(list('ACGT'), L + K - 1))
+        means = rs.normal(size=L + K - 1)
+        args = (int(rs.randint(0, 50)),)
+        reg_start = int(rs.randint(0, 60))
+        args += (reg_start, reg_start + int(rs.randint(1, 60)), str(rs.choice(['+', '-'])), K, cp,
+                 int(rs.randint(0, 4)), int(rs.randint(0, 8)))
+        yield seq, means, args
+
+
+def trim_result(fn, err, seq, means, args):
+    """fn(seq, means, *args) as plain values: ('ok', kmers, means, r_start, motif seq) or
+    ('err', message) for an exception of type err."""
+    try:
+        k, mm, r, ms = fn(seq, means.copy(), *args)
+        return ('ok', [str(x) for x in k], [float(x) for x in mm], int(r), str(ms))
+    except err as e:
+        return ('err', str(e))
+
+
+def stall_cases():
+    """1000 seeded (stall intervals, sorted change points) pairs for remove_stall_cpts."""
+    rs = np.random.RandomState(4)
+    for _ in range(1000):
+        ns = int(rs.randint(0, 6))
+        ints = np.sort(rs.choice(np.arange(0, 2000), 2 * ns, replace=False)).reshape(-1, 2)
+        cp = np.sort(rs.choice(np.arange(0, 2000), int(rs.randint(1, 300)),
+                               replace=False)).astype(np.int64)
+        yield [tuple(int(v) for v in x) for x in ints], cp

@@ -61,28 +61,24 @@ def test_python_api_surface_imports_without_gpu():
 
 
 def test_parameters_and_namedtuples_match_reference_when_available():
-    import sys, os
-    sys.path.insert(0, os.path.join(REPO, 'oracle'))
-    import ref_harness as rh
-    if not rh.available():
-        pytest.skip('oracle/_ref not built')
-    m = rh.load_reference()
+    """against the reference's values, recorded by tests/golden/make_reference_api_golden.py"""
+    import ast
+    import json
     from tombo_b200 import tombo_helper as th, tombo_stats as ts, _default_parameters as dp
-    import tombo._default_parameters as rdp
+    g = json.load(open(os.path.join(REPO, 'tests', 'golden', 'reference_api.json')))
+    ref = {n: ast.literal_eval(v) for n, v in g['default_parameters'].items()}
     for name in dir(dp):
         if name.isupper():
-            assert getattr(dp, name) == getattr(rdp, name), name
-    for nt in ('alignInfo', 'readData', 'scaleValues', 'resquiggleParams', 'resquiggleResults',
-               'dpResults', 'genomeLocation', 'seqSampleType', 'stallParams', 'channelInfo'):
-        assert getattr(th, nt)._fields == getattr(m['th'], nt)._fields, nt
-    for kind in ('DNA', 'RNA'):
+            assert name in ref and getattr(dp, name) == ref[name], name
+    assert len(g['namedtuple_fields']) == 10
+    for nt, fields in g['namedtuple_fields'].items():
+        assert getattr(th, nt)._fields == tuple(fields), nt
+    assert len(g['resquiggle_parameters']) == 4
+    for kind, save, b in g['resquiggle_parameters']:
         sst = th.seqSampleType(kind, kind == 'RNA')
-        for save in (False, True):
-            a = ts.load_resquiggle_parameters(sst, use_save_bandwidth=save)
-            b = m['ts'].load_resquiggle_parameters(m['th'].seqSampleType(kind, kind == 'RNA'),
-                                                   use_save_bandwidth=save)
-            assert tuple(a) == tuple(b)
-    assert ts.HALF_NORM_EXPECTED_VAL == m['ts'].HALF_NORM_EXPECTED_VAL
+        a = ts.load_resquiggle_parameters(sst, use_save_bandwidth=save)
+        assert tuple(a) == ast.literal_eval(b), (kind, save)
+    assert ts.HALF_NORM_EXPECTED_VAL == ast.literal_eval(g['half_norm_expected_val'])
 
 
 def test_pipeline_chunk_schedule_covers_every_read_once():

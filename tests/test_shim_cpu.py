@@ -1,8 +1,11 @@
 """CPU: host-side pieces of the Python mirror API -- batch packing (one bad read never
 aborts a batch), error typing, and the two helpers re-expressed in vectorised form checked
-against the unmodified reference (oracle/_ref) on random inputs."""
+against the unmodified reference on random inputs (digests of its outputs recorded by
+tests/golden/make_reference_api_golden.py)."""
 import numpy as np
 import pytest
+
+import golden_util as gu
 
 
 def _map_res(raw, seq):
@@ -51,53 +54,25 @@ def test_batcher_files_library_errors_as_non_tombo():
     assert out[2][1][0] is False
 
 
-def _reference():
-    import ref_harness as rh
-    if not rh.available():
-        pytest.skip('oracle/_ref not built')
-    return rh.load_reference()
-
-
 def test_trim_seq_and_means_equals_reference_on_random_regions():
-    m = _reference()
     from tombo_b200 import tombo_stats as ts, tombo_helper as th
-    rs = np.random.RandomState(3)
-    seen = {'ok': 0, 'err': 0}
-    for it in range(3000):
-        K = int(rs.choice([5, 6, 7])); cp = int(rs.randint(0, K))
-        L = int(rs.randint(K, 40))
-        seq = ''.join(rs.choice(list('ACGT'), L + K - 1))
-        means = rs.normal(size=L + K - 1)
-        args = (int(rs.randint(0, 50)),)
-        reg_start = int(rs.randint(0, 60))
-        args += (reg_start, reg_start + int(rs.randint(1, 60)), str(rs.choice(['+', '-'])), K, cp,
-                 int(rs.randint(0, 4)), int(rs.randint(0, 8)))
-
-        def call(f, err):
-            try:
-                k, mm, r, ms = f(seq, means.copy(), *args)
-                return ('ok', list(k), mm.tolist(), r, ms)
-            except err as e:
-                return ('err', str(e))
-        a = call(m['ts'].trim_seq_and_means, m['th'].TomboError)
-        b = call(ts.trim_seq_and_means, th.TomboError)
-        assert a == b, (it, args)
-        seen[a[0]] += 1
-    assert seen['ok'] > 500 and seen['err'] > 500
+    g = gu.load('reference_api')
+    ok, dig = g['trim_ok'], g['trim_digest']
+    assert ok.shape[0] == dig.shape[0] == 3000
+    for it, (seq, means, args) in enumerate(gu.trim_cases()):
+        b = gu.trim_result(ts.trim_seq_and_means, th.TomboError, seq, means, args)
+        assert (b[0] == 'ok') == bool(ok[it]), (it, args, b)
+        assert np.array_equal(gu.digest(b), dig[it]), (it, args, b)
+    assert ok.sum() > 500 and (~ok).sum() > 500
 
 
 def test_remove_stall_cpts_equals_reference():
-    m = _reference()
     from tombo_b200 import resquiggle as rq
-    rs = np.random.RandomState(4)
-    for it in range(1000):
-        ns = int(rs.randint(0, 6))
-        ints = np.sort(rs.choice(np.arange(0, 2000), 2 * ns, replace=False)).reshape(-1, 2)
-        cp = np.sort(rs.choice(np.arange(0, 2000), int(rs.randint(1, 300)),
-                               replace=False)).astype(np.int64)
-        a = m['ts'].remove_stall_cpts([tuple(x) for x in ints], cp)
-        b = rq._remove_stall_cpts([tuple(x) for x in ints], cp)
-        assert np.array_equal(a, b)
+    dig = gu.load('reference_api')['stall_digest']
+    assert dig.shape[0] == 1000
+    for it, (ints, cp) in enumerate(gu.stall_cases()):
+        b = np.asarray(rq._remove_stall_cpts(ints, cp), dtype=np.int64).tolist()
+        assert np.array_equal(gu.digest(b), dig[it]), (it, ints)
 
 
 def test_write_new_fast5_group_opens_path_likes_and_always_closes(monkeypatch, tmp_path):
